@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the gsx hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gsx|reference] [--config c2|c3|c4|c5] [--splats-per-gpu N]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Default (`--config c2`, the driver's contract line).  Metric: Msplats/s of Statistical Outlier Removal, k=16,
@@ -61,7 +62,14 @@ def parse():
     ap.add_argument("--hash", default="i32wrap", choices=["i32wrap", "i64"])
     ap.add_argument("--cpu-sample", type=int, default=1_000_000, help="points of the in-line CPU-baseline sample")
     ap.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / e2e / kmeans / parity extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy "
+                         "(--config c2, --impl gsx; see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and (a.impl != "gsx" or a.config != "c2"):
+        ap.error("--dump-outputs is defined for --impl gsx --config c2")
     if a.n is None:
         a.n = {"c2": 10_000_000, "c3": 50_000_000, "c4": 50_000_000, "c5": 125_000_000}[a.config]
     return a
@@ -377,6 +385,33 @@ def sog_schedule(n_rows, level=5):
     return num_chunks, chunk, max(16, int(np.ceil(target_k / num_chunks)))
 
 
+DUMP_SAMPLE = 1 << 21   # points of the dumped sample: 32 MiB of .npy files at most
+
+
+def dump_outputs(out_dir: Path, mask, means=None):
+    """What a caller of the c2 path receives from one step -- the keep-mask and (one GPU) the SOR mean distances --
+    as .npy files, so that two builds can be compared output for output.  Above DUMP_SAMPLE points, the same seeded
+    sample of point indices is written every run (`sample_index`).  `keep_count` (masked points of the whole cloud)
+    and `mean_std` (the threshold statistics over all mean distances) cover every point."""
+    import torch
+    from gsx import sor
+    n = mask.numel()
+    if n > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    else:
+        idx = np.arange(n)
+    idx_d = torch.from_numpy(idx).to(mask.device)
+    out = {"sample_index": idx.astype(np.float64),
+           "keep_mask": mask[idx_d].cpu().numpy().astype(np.float32),
+           "keep_count": np.array([int(mask.sum())], dtype=np.float64)}
+    if means is not None:
+        out["mean_dists"] = means[idx_d].cpu().numpy()
+        out["mean_std"] = sor.mean_std(means).cpu().numpy()
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 # ----------------------------------------------------------------------------- c2: the contract line
 def run_c2(args):
     import torch
@@ -431,6 +466,8 @@ def run_c2(args):
     barrier(world)
     clocks.window_end()
     launches = _abi.lib.gsx_kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:       # before the busy steps below reuse `means`
+        dump_outputs(Path(args.dump_outputs), mask, means if world == 1 else None)
     clk = finish_clocks(clocks, world, rank, dev, lambda: step(False))
     elapsed_ms = max_over_ranks(t_start.elapsed_time(t_end), dev, world)
     ms_per_step = elapsed_ms / args.steps

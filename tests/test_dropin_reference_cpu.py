@@ -1,13 +1,15 @@
-"""CPU (this container only): gsx.dropin.patch() against the REAL reference tree (/root/reference, imported read-only
-with a stub `plyfile`).  The GPU box has no /root/reference and this container has no GPU, so the device layer
-(gsx.pipeline.FilterChain, gsx.kmeans host entry points) is replaced by oracle-backed stand-ins; everything between
-the reference's call sites and that layer is the shipped code: the patched gsconverter.processing.{DataProcessor,
-gpu_ops}, the converter.py:194-236 filter chain, SogFormat.write with its K-Means call shapes, the batch-ahead of the
-shN chunk loop and its RNG transparency.  Checks:
-  * bbox / alpha / density outputs of the patched chain == the UNPATCHED reference's own outputs;
+"""CPU: gsx.dropin.patch() on a `gsconverter` package, checked against what the reference 3dgsconverter computes on
+the same records (tests/golden/g10_reference_dropin.npz, recorded by tests/golden/make_reference_records.py).
+The patch is applied to this repository's own `gsconverter` package, and the device layer (gsx.pipeline.FilterChain,
+the gsx.kmeans host entry points) is replaced by oracle-backed stand-ins so that the test needs no GPU; everything
+between the package's call sites and that layer is the shipped code: the patched gsconverter.processing.
+{DataProcessor, gpu_ops}, the converter.py:194-236 filter chain, and the batch-ahead of the SOG shN chunk loop with its
+RNG transparency.  Checks:
+  * bbox / alpha / density outputs of the patched chain == the UNPATCHED reference's outputs (SHA-256 of the records);
   * SOR through the patch == the oracle's Taichi-semantics mask (the reference's own CPU path discards its mask, F5);
-  * SogFormat.write: the 64-chunk loop reaches the backend as ONE batched launch, K-Means call shapes follow
-    sog.py:392-552, and the written archive is byte-identical with batch-ahead on and off (same seed).
+  * the reference SogFormat.write's sequence of gpu_ops.kmeans calls, replayed through the patched gpu_ops: the
+    shN chunk loop reaches the backend as ONE batched launch, the call shapes follow sog.py:392-552, and every result
+    and the global RNG stream are bit-identical with batch-ahead on and off (same seed).
 """
 import json
 import os
@@ -16,29 +18,24 @@ import sys
 import textwrap
 from pathlib import Path
 
-import pytest
-
 ROOT = Path(__file__).resolve().parent.parent
-REF = Path("/root/reference")
-
-pytestmark = pytest.mark.skipif(not (REF / "gsconverter").exists(), reason="needs the reference tree at /root/reference")
+GOLD = ROOT / "tests" / "golden" / "g10_reference_dropin.npz"
 
 DRIVER = textwrap.dedent(r'''
-    import hashlib, io, json, os, sys, tempfile, types, zipfile
+    import hashlib, json, sys
     import numpy as np
-    ROOT, REF = sys.argv[1], sys.argv[2]
-    sys.path[:0] = [REF, ROOT, ROOT + "/3dgsconverter_b200"]          # `gsconverter` = the reference; `gsx` = ours
-    ply = types.ModuleType("plyfile"); ply.PlyData = ply.PlyElement = object; sys.modules["plyfile"] = ply
-    import gsconverter                                                 # the real reference package
-    assert gsconverter.__file__.startswith(REF), gsconverter.__file__
-    from gsconverter.processing.data_processor import DataProcessor as RefDP
-    from gsconverter.formats.sog import SogFormat
-    import gsconverter.formats.sog as ref_sog
+    ROOT, GOLD = sys.argv[1], sys.argv[2]
+    sys.path[:0] = [ROOT, ROOT + "/3dgsconverter_b200"]
+    import gsconverter                                                 # this repository's package
+    assert gsconverter.__file__.startswith(ROOT + "/3dgsconverter_b200/"), gsconverter.__file__
+    from gsconverter.processing.data_processor import DataProcessor as UnpatchedDP
     import oracle
     import gsx, gsx.pipeline, gsx.kmeans, gsx.dropin
     from gsx import synth
+    ref = np.load(GOLD)
+    sha = lambda a: hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
-    # ---------------- oracle-backed stand-ins for the device layer (no GPU in this container)
+    # ---------------- oracle-backed stand-ins for the device layer (no GPU needed)
     calls = {"kmeans_host": [], "kmeans_host_batched": []}
 
     class OracleChain:
@@ -88,37 +85,35 @@ DRIVER = textwrap.dedent(r'''
     gsx.backend_available = lambda: True
     gsx.dropin.backend_available = gsx.backend_available if hasattr(gsx.dropin, "backend_available") else None
 
-    N = int(sys.argv[3])
-    data = synth.structured(N, "mixed")
+    data = synth.structured(100_000, "mixed")
     out = {}
 
-    # ---------------- 1. the UNPATCHED reference on the same records (its own NumPy paths)
-    ref = RefDP(data.copy())
-    r_bbox = ref.crop_by_bbox(-11, -11, -11, 11, 11, 11).copy()
-    r_alpha = ref.apply_alpha_filter(5).copy()
-    r_dens = ref.apply_density_filter(1.0, 0.32, sensitivity=0.5, keep_multicluster=True).copy()
-
-    # ---------------- 2. patch and run the converter.py:194-236 chain through gsconverter.processing
+    # ---------------- 1. patch and run the converter.py:194-236 chain through gsconverter.processing
     assert gsx.dropin.patch(defer=True) is True
     import gsconverter.processing as proc
     from gsconverter.processing import gpu_ops
     assert gpu_ops._GSX_PATCHED and gpu_ops.HAS_TAICHI is True
     P = proc.DataProcessor
-    assert P is not RefDP and P.__module__.endswith("_gsx_data_processor")
+    assert P is not UnpatchedDP and P.__module__.endswith("_gsx_data_processor")
     dp = P(data.copy())
     dp.crop_by_bbox(-11, -11, -11, 11, 11, 11); p_bbox = dp.data.copy()
     dp.apply_alpha_filter(5); p_alpha = dp.data.copy()
     dp.apply_density_filter(1.0, 0.32, sensitivity=0.5, keep_multicluster=True); p_dens = dp.data.copy()
     dp.remove_flyers(16, 2.0); p_sor = dp.data.copy()
-    out["bbox_equal"] = bool(np.array_equal(r_bbox, p_bbox))
-    out["alpha_equal"] = bool(np.array_equal(r_alpha, p_alpha))
-    out["density_equal"] = bool(np.array_equal(r_dens, p_dens))
-    xyz_d = np.column_stack((r_dens["x"], r_dens["y"], r_dens["z"]))
+    # ---------------- 2. against the UNPATCHED reference on the same records (its own NumPy paths)
+    out["bbox_equal"] = sha(p_bbox) == str(ref["bbox_sha"])
+    out["alpha_equal"] = sha(p_alpha) == str(ref["alpha_sha"])
+    out["density_equal"] = sha(p_dens) == str(ref["density_sha"])
+    xyz_d = np.column_stack((p_dens["x"], p_dens["y"], p_dens["z"]))
     want = oracle.sor_taichi_mask(xyz_d, 16, 2.0, "i32wrap")
-    out["sor_equal_oracle"] = bool(np.array_equal(r_dens[want], p_sor))
-    out["counts"] = [len(r_bbox), len(r_alpha), len(r_dens), len(p_sor)]
+    out["sor_equal_oracle"] = bool(np.array_equal(p_dens[want], p_sor))
+    out["counts"] = [len(p_bbox), len(p_alpha), len(p_dens), len(p_sor)]
+    out["ref_counts"] = ref["counts"].tolist()
 
-    # ---------------- 3. SogFormat.write through the patch: call shapes, one batched launch, RNG transparency
+    # ---------------- 3. the reference SogFormat.write's gpu_ops.kmeans calls through the patch: call shapes, one
+    # batched launch, RNG transparency.  The shN chunks are row ranges of one block of the survivors' SH rows, as in
+    # the writer; the other inputs come from a generator of their own, outside the global RNG.
+    block = np.ascontiguousarray(np.column_stack([p_sor[f"f_rest_{i}"] for i in range(45)]), dtype=np.float32)
     def write(batch_ahead):
         g = gpu_ops._gsx_module
         g.BATCH_AHEAD = batch_ahead
@@ -126,38 +121,42 @@ DRIVER = textwrap.dedent(r'''
         for k in g.batch_stats: g.batch_stats[k] = 0
         calls["kmeans_host"].clear(); calls["kmeans_host_batched"].clear()
         np.random.seed(4242)
-        path = tempfile.mktemp(suffix=".sog")
-        SogFormat().write(p_sor.copy(), path, compression_level=5)
-        zf = zipfile.ZipFile(path)
-        digest = {n: hashlib.sha256(zf.read(n)).hexdigest() for n in sorted(zf.namelist()) if not n.startswith("shN_centroids") and n != "meta.json"}
-        meta = json.loads(zf.read("meta.json"))
-        os.unlink(path)
-        return digest, meta, dict(g.batch_stats), list(calls["kmeans_host"]), list(calls["kmeans_host_batched"]), np.random.get_state()[1][:8].tolist()
-    d_on, meta_on, st_on, single_on, batched_on, rng_on = write(True)
-    d_off, meta_off, st_off, single_off, batched_off, rng_off = write(False)
+        digests = []
+        for i, (rows, cols, k, max_iter, start, base_rows, rng_moved) in enumerate(ref["sog_kmeans_calls"].tolist()):
+            if rng_moved:
+                np.random.random()            # the writer drew from the global RNG since the previous call
+            if start >= 0:
+                assert base_rows == len(block) and cols == 45, (base_rows, len(block))
+                d = block[start:start + rows]
+            else:
+                d = np.random.default_rng(i).standard_normal((rows, cols), dtype=np.float32)
+            C, L = gpu_ops.kmeans(d, k, max_iter=max_iter)
+            digests.append((sha(C), sha(L)))
+        return digests, dict(g.batch_stats), list(calls["kmeans_host"]), list(calls["kmeans_host_batched"]), np.random.get_state()[1].tolist()
+    d_on, st_on, single_on, batched_on, rng_on = write(True)
+    d_off, st_off, single_off, batched_off, rng_off = write(False)
     n_s = len(p_sor)
     num_chunks = max(1, min(64, n_s // 1024)); chunk = int(np.ceil(n_s / num_chunks))
-    out["sog"] = {"files_equal_batch_on_off": d_on == d_off, "labels_file_present": "shN_labels.webp" in d_on,
+    out["sog"] = {"results_equal_batch_on_off": d_on == d_off,
                   "stats_on": st_on, "stats_off": st_off, "batched_calls_on": batched_on, "single_calls_on": single_on[:4],
                   "single_calls_off_shN": [c for c in single_off if c[0][1] == 45][:2], "n_single_off_shN": len([c for c in single_off if c[0][1] == 45]),
-                  "num_chunks": num_chunks, "chunk": chunk, "n": n_s, "shN_count_on": meta_on["shN"]["count"], "shN_count_off": meta_off["shN"]["count"],
-                  "rng_after_equal": rng_on == rng_off,
-                  "scales_codebook_equal": meta_on["scales"]["codebook"] == meta_off["scales"]["codebook"]}
+                  "num_chunks": num_chunks, "chunk": chunk, "n": n_s,
+                  "rng_after_equal": rng_on == rng_off}
     print("RESULT " + json.dumps(out))
 ''')
 
 
-def test_patch_against_the_real_reference(tmp_path):
+def test_patch_against_the_real_reference(tmp_path, gsx_lib):
     drv = tmp_path / "driver.py"
     drv.write_text(DRIVER)
     env = dict(os.environ, OMP_NUM_THREADS="8", PYTHONWARNINGS="ignore")
-    r = subprocess.run([sys.executable, str(drv), str(ROOT), str(REF), "100000"], capture_output=True, text=True,
+    r = subprocess.run([sys.executable, str(drv), str(ROOT), str(GOLD)], capture_output=True, text=True,
                        timeout=1500, env=env)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
     line = [ln for ln in r.stdout.splitlines() if ln.startswith("RESULT ")][-1]
     out = json.loads(line[7:])
     assert out["bbox_equal"] and out["alpha_equal"] and out["density_equal"], out
-    assert out["sor_equal_oracle"], out
+    assert out["sor_equal_oracle"] and out["counts"] == out["ref_counts"], out
     sog = out["sog"]
     # sog.py:392-445: two 1-D fits on <= 50 000 scalars, K=256, max_iter=20 -- single calls in both modes
     assert sog["single_calls_on"][:2] == [[[50000, 1], 256, 20], [[50000, 1], 256, 20]], sog
@@ -168,5 +167,4 @@ def test_patch_against_the_real_reference(tmp_path):
     assert len(sog["batched_calls_on"]) == 1 and sog["batched_calls_on"][0][1] == sog["num_chunks"], sog
     assert sog["batched_calls_on"][0][0] == [sog["n"], 45], sog
     # identical results and identical global RNG stream either way
-    assert sog["files_equal_batch_on_off"] and sog["rng_after_equal"] and sog["scales_codebook_equal"], sog
-    assert sog["shN_count_on"] == sog["shN_count_off"], sog
+    assert sog["results_equal_batch_on_off"] and sog["rng_after_equal"], sog

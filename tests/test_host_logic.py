@@ -99,6 +99,37 @@ def test_bench_reference_arm_does_not_load_libgsx():
     assert out.returncode == 0, out.stderr[-2000:]
 
 
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "d"],
+                                  ["--config", "c3", "--dump-outputs", "d"]])
+def test_bench_rejects_arguments_it_cannot_honour(argv, tmp_path):
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), *argv], capture_output=True, text=True, timeout=120,
+                         cwd=tmp_path)
+    assert out.returncode == 2 and "error:" in out.stderr, out.stderr[-2000:]
+    assert not (tmp_path / "d").exists()
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_the_timed_step_results(cuda, gsx_lib, tmp_path):
+    """`bench.py --dump-outputs DIR`: the last timed step's keep-mask and mean distances, equal to the oracle's."""
+    from gsx import synth
+    n = 200_000
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1",
+                          "--no-extras", "--splats-per-gpu", str(n), "--dump-outputs", str(tmp_path / "d")],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 3 and line["warmup"] == 1
+    d = {p.stem: np.load(p) for p in (tmp_path / "d").glob("*.npy")}
+    assert set(d) == {"sample_index", "keep_mask", "keep_count", "mean_dists", "mean_std"}
+    assert all(a.dtype in (np.float32, np.float64) for a in d.values())
+    assert sum(p.stat().st_size for p in (tmp_path / "d").glob("*.npy")) <= 64 << 20
+    assert np.array_equal(d["sample_index"], np.arange(n))        # below the sample size: every point
+    want = oracle.sor_taichi_mean_dists(synth.xyz(n, "mixed"), 16, "i32wrap")
+    assert np.array_equal(d["mean_dists"].view(np.uint32), want.view(np.uint32))
+    mask = oracle.threshold_mask(want, 2.0)
+    assert np.array_equal(d["keep_mask"], mask.astype(np.float32)) and d["keep_count"][0] == mask.sum() == line["run"]["kept"]
+
+
 def test_dropin_mirror_has_reference_surface():
     """Names and signatures of the plugin surface (SURVEY §8b) -- importable without a GPU."""
     import inspect

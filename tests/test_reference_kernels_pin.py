@@ -1,22 +1,20 @@
 """The pin for the Taichi-semantics SOR and the Lloyd K-Means: outputs of the REFERENCE'S OWN kernel source.
 
-tests/golden/g4_reference_kernels.npz was produced by executing /root/reference/gsconverter/processing/gpu_ops.py
+tests/golden/g4_reference_kernels.npz was produced by executing the reference's gsconverter/processing/gpu_ops.py
 (unmodified: filter_sor_gpu :193-263 with kernel :98-176, _kmeans_taichi :178-191 with kernels :57-96) under the
 serial `taichi` stand-in of tests/golden/ti_serial.py (assumptions T1-T5 in its header), by
 tests/golden/make_taichi_goldens.py.  Bar: mean distances, keep-masks, labels and centroids bit-identical.
 
-  * CPU (`-m "not gpu"`): the oracle against the fixture; the stand-in really runs the reference's text (live, when
-    /root/reference exists -- it does not on the GPU box);
+  * CPU (`-m "not gpu"`): the oracle against the fixtures (g9: a small run of the reference's text under the
+    stand-in, recorded by tests/golden/make_reference_records.py);
   * GPU (`-m gpu`): the CUDA path, through the C ABI and through the drop-in plugin functions, against the fixture.
 """
-import os
 from pathlib import Path
 
 import numpy as np
 import pytest
 
 GOLD = Path(__file__).resolve().parent / "golden" / "g4_reference_kernels.npz"
-REF = "/root/reference/gsconverter/processing/gpu_ops.py"
 
 
 def _sor_cases(g):
@@ -88,30 +86,24 @@ def test_oracle_reproduces_reference_kmeans_kernels():
         assert np.array_equal(Co.view(np.uint32), C.view(np.uint32)), name
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="needs /root/reference (build container only)")
-def test_stand_in_executes_the_reference_source_live():
-    """A small live run: the reference's file, loaded by path with the stand-in, against the oracle; and the text the
-    stand-in compiled is the reference's kernel body (typed literals aside)."""
-    import sys
-    sys.path.insert(0, str(GOLD.parent))
-    import ti_serial
+G9 = GOLD.parent / "g9_reference_small_run.npz"
+
+
+def test_oracle_reproduces_recorded_reference_source_run():
+    """g9 (make_reference_records.py): a small run of the reference's file, loaded by path with the stand-in (the
+    generator also asserts that the text the stand-in compiled is the reference's kernel body); the oracle reproduces
+    the SOR keep-mask and the K-Means labels and centroids bit for bit."""
     import oracle
-    ref = ti_serial.import_reference_gpu_ops()
-    src = ref.sor_compute_mean_dists.__ti_serial_source__
-    for fragment in ("h = (nx * p1 ^ ny * p2 ^ nz * p3) % hash_size", "while ins_pos >", "d = ti.sqrt(d2)",
-                     "mean_dists[i] = sum_d / _ti_f32cast(valid_k)"):
-        assert fragment in src, fragment
-    assert "centroids[l, dim] += data[i, dim]" in ref.k_means_update.__ti_serial_source__   # ti.atomic_add, serial (T4)
+    g = np.load(G9)
     rng = np.random.default_rng(3)
     xyz = np.concatenate([rng.normal(0, 0.05, (250, 3)), rng.uniform(-2, 2, (150, 3))]).astype(np.float32)
-    mask = ref.filter_sor_gpu(xyz, k=12, threshold_factor=1.5)
+    mask = g["sor_mask"]
+    assert mask.dtype == bool and 0 < mask.sum() < len(xyz)
     assert np.array_equal(mask, oracle.sor_taichi_mask(xyz, 12, 1.5, "i32wrap"))
     X = rng.normal(size=(300, 5)).astype(np.float32)
     np.random.seed(11)
-    C, L = ref._kmeans_taichi(X, 7, max_iter=3)
-    np.random.seed(11)
     Co, Lo, _ = oracle.kmeans_lloyd(X, 7, 3, init=X[np.random.choice(300, 7, replace=False)])
-    assert np.array_equal(L, Lo) and np.array_equal(C.view(np.uint32), Co.view(np.uint32))
+    assert np.array_equal(g["km_labels"], Lo) and np.array_equal(g["km_centroids"].view(np.uint32), Co.view(np.uint32))
 
 
 # ---- BASELINE configs[0]: the 100 k cloud, --sor_intensity 5 (k=27) and k=16, through the reference's source
