@@ -102,12 +102,22 @@ int gsx_device_sm_count(void) {
 
 /* ------------------------------------------------------------------ SOR */
 
-int64_t gsx_sor_workspace_bytes(int64_t n) { return sor_workspace_bytes(n); }
-int64_t gsx_sor_grid_workspace_bytes(int64_t n) { return sor_grid_workspace_bytes(n); }
+// The workspace sizes of the entry points bounded by GSX_N_LIMIT refuse what those entry points refuse.
+#define GSX_WS_LIMIT(what, n)                                                                                    \
+    GSX_REQUIRE((n) < GSX_N_LIMIT, GSX_ERR_ARG, what ": n=%lld out of range [0, 2^31-64)", (long long)(n))
+
+int64_t gsx_sor_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("sor", n);
+    return sor_workspace_bytes(n);
+}
+int64_t gsx_sor_grid_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("sor", n);
+    return sor_grid_workspace_bytes(n);
+}
 
 // grid-only functions (build_from_sorted, mean_dists) accept the shorter gsx_sor_grid_workspace_bytes blob
 static int carve_grid_checked(void* ws, int64_t ws_bytes, int64_t n, SorWs& w) {
-    GSX_REQUIRE(n >= 1 && n < 2147483584ll, GSX_ERR_ARG, "sor: n=%lld out of range [1, 2^31-64)", (long long)n);
+    GSX_REQUIRE(n >= 1 && n < GSX_N_LIMIT, GSX_ERR_ARG, "sor: n=%lld out of range [1, 2^31-64)", (long long)n);
     GSX_REQUIRE(ws != nullptr, GSX_ERR_WORKSPACE, "sor: null workspace");
     w = sor_carve(ws, ws_bytes, n, sor_sort_ws_bytes(n));
     GSX_REQUIRE(w.grid_ok, GSX_ERR_WORKSPACE, "sor: grid workspace too small (%lld < %zu)", (long long)ws_bytes,
@@ -116,7 +126,7 @@ static int carve_grid_checked(void* ws, int64_t ws_bytes, int64_t n, SorWs& w) {
 }
 
 static int carve_checked(void* ws, int64_t ws_bytes, int64_t n, SorWs& w) {
-    GSX_REQUIRE(n >= 1 && n < 2147483584ll, GSX_ERR_ARG, "sor: n=%lld out of range [1, 2^31-64)", (long long)n);
+    GSX_REQUIRE(n >= 1 && n < GSX_N_LIMIT, GSX_ERR_ARG, "sor: n=%lld out of range [1, 2^31-64)", (long long)n);
     GSX_REQUIRE(ws != nullptr, GSX_ERR_WORKSPACE, "sor: null workspace");
     w = sor_carve(ws, ws_bytes, n, sor_sort_ws_bytes(n));
     GSX_REQUIRE(w.ok, GSX_ERR_WORKSPACE, "sor: workspace too small (%lld < %zu)", (long long)ws_bytes, w.total);
@@ -173,7 +183,7 @@ int gsx_sor_dist_local_run(const float* xyz_local_dev, int64_t n_local, int64_t 
     SorWs w;
     int rc = carve_checked(ws, ws_bytes, n_local > 0 ? n_local : 1, w);
     if (rc) return rc;
-    GSX_REQUIRE(n_global >= n_local && n_global >= 1 && n_global < 2147483584ll, GSX_ERR_ARG, "sor: bad n_global");
+    GSX_REQUIRE(n_global >= n_local && n_global >= 1 && n_global < GSX_N_LIMIT, GSX_ERR_ARG, "sor: bad n_global");
     return sor_dist_local_run(xyz_local_dev, n_local, idx_base, n_global, world, bmin_host, cell,
                               (float4*)pos4_out_dev, (long long*)cuts_dev, w, (cudaStream_t)stream);
 }
@@ -278,7 +288,7 @@ int gsx_sor_filter_device(const float* xyz_dev, int64_t n, int32_t k, float thre
 
 int gsx_sor_filter_host(const float* xyz_host, int64_t n, int32_t k, float threshold_factor, int32_t hash_mode,
                         uint8_t* mask_host, float* means_host) {
-    GSX_REQUIRE(n >= 1 && n < 2147483584ll, GSX_ERR_ARG, "sor: n=%lld out of range", (long long)n);
+    GSX_REQUIRE(n >= 1 && n < GSX_N_LIMIT, GSX_ERR_ARG, "sor: n=%lld out of range", (long long)n);
     cudaStream_t st = 0;
     int64_t wsb = sor_workspace_bytes(n);
     DevBuf xyz(st), ws(st), mask(st), means(st);
@@ -303,6 +313,7 @@ int gsx_sor_filter_host(const float* xyz_host, int64_t n, int32_t k, float thres
 /* ------------------------------------------------------------------ pair sort (gpu_ops.py:227) */
 
 int64_t gsx_sort_pairs_workspace_bytes(int64_t n) {
+    GSX_REQUIRE(n < (1ll << 32), GSX_ERR_ARG, "sort: n=%lld out of range [0, 2^32)", (long long)n);
     if (n < 1) n = 1;
     return (int64_t)(align_up((size_t)n * 8, 256) + align_up((size_t)n * 4, 256) + radix_ws_bytes(n) + 1024);
 }
@@ -330,7 +341,10 @@ int gsx_sort_pairs(uint64_t* keys_dev, int32_t* vals_dev, int64_t n, int32_t beg
 
 /* ------------------------------------------------------------------ SOR, cKDTree semantics */
 
-int64_t gsx_knn_exact_workspace_bytes(int64_t n) { return knn_exact_workspace_bytes(n); }
+int64_t gsx_knn_exact_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("knn_exact", n);
+    return knn_exact_workspace_bytes(n);
+}
 
 int gsx_knn_exact_mean_dists(const float* xyz_dev, int64_t n, int32_t k, float* means_dev, void* ws, int64_t ws_bytes,
                              void* stream) {
@@ -339,7 +353,7 @@ int gsx_knn_exact_mean_dists(const float* xyz_dev, int64_t n, int32_t k, float* 
 
 int gsx_sor_ckdtree_filter_host(const float* xyz_host, int64_t n, int32_t k, float threshold_factor, uint8_t* mask_host,
                                 float* means_host) {
-    GSX_REQUIRE(n >= 1 && n < 2147483584ll, GSX_ERR_ARG, "sor: n=%lld out of range", (long long)n);
+    GSX_REQUIRE(n >= 1 && n < GSX_N_LIMIT, GSX_ERR_ARG, "sor: n=%lld out of range", (long long)n);
     cudaStream_t st = 0;
     int64_t wsb = knn_exact_workspace_bytes(n);
     int64_t msb = (int64_t)mean_std_ws_bytes(n);
@@ -386,7 +400,10 @@ double gsx_alpha_logit_threshold(double min_opacity_u8) {
 
 /* ------------------------------------------------------------------ compaction between filters */
 
-int64_t gsx_compact_workspace_bytes(int64_t n) { return compact_workspace_bytes(n); }
+int64_t gsx_compact_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("compact", n);
+    return compact_workspace_bytes(n);
+}
 
 int gsx_compact_points(const uint8_t* mask_dev, int64_t n, const float* xyz_dev, const float* opacity_dev,
                        const int32_t* idx_dev, float* xyz_out_dev, float* opacity_out_dev, int32_t* idx_out_dev,
@@ -430,7 +447,10 @@ int gsx_density_grid_dense(const int32_t* grid_dev, const int64_t* q0, const int
 
 /* ------------------------------------------------------------------ SOG writer helpers (SURVEY 8f-1) */
 
-int64_t gsx_lexsort_workspace_bytes(int64_t n) { return lexsort_workspace_bytes(n); }
+int64_t gsx_lexsort_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("lexsort", n);
+    return lexsort_workspace_bytes(n);
+}
 
 int gsx_lexsort_zyx(const float* xyz_dev, int64_t n, int32_t* order_dev, void* ws, int64_t ws_bytes, void* stream) {
     return lexsort_zyx(xyz_dev, n, order_dev, ws, ws_bytes, (cudaStream_t)stream);
@@ -558,7 +578,10 @@ int gsx_records_scale_exp(const float* rows_dev, int64_t n, int32_t F, int32_t s
 }
 
 /* ------------------------------------------------------------------ Morton ordering primitive (SURVEY 8f 3) */
-int64_t gsx_morton_workspace_bytes(int64_t n) { return morton_workspace_bytes(n); }
+int64_t gsx_morton_workspace_bytes(int64_t n) {
+    GSX_WS_LIMIT("morton", n);
+    return morton_workspace_bytes(n);
+}
 int gsx_morton_order(const float* xyz_dev, int64_t n, int32_t* order_dev, int32_t run_limit, int32_t* levels_out, void* ws,
                      int64_t ws_bytes, void* stream) {
     int lv = 0;

@@ -8,6 +8,7 @@
 // (64 M rows, 50 % survivors): count -> multi-level scan -> scatter (0.72 ms) and the shipped single pass with
 // decoupled look-back over per-tile survivor counts (k_cmp_onepass, 0.66 ms).  A first single-pass version that staged
 // the survivors' DATA in 40 KiB of shared memory per block was slower than both (0.85 ms: occupancy).
+#include "../../include/gsx.h"
 #include "gsx_common.cuh"
 #include "gsx_compact.cuh"
 #include "gsx_radix.cuh"
@@ -66,6 +67,14 @@ __global__ void __launch_bounds__(kCmpBlock)
 #ifndef GSX_COMPACT_ONEPASS
 #define GSX_COMPACT_ONEPASS 1   // single pass with decoupled look-back; 0 = the count -> scan -> scatter form (A/B)
 #endif
+// The single pass handles n < GSX_COMPACT_ONEPASS_MAX_N: its look-back words carry the running survivor count in 30
+// bits, so from 2^30 rows on (2^30 survivors are possible) the count -> scan -> scatter form runs, whose 32-bit block
+// offsets hold any n < 2^31.  A smaller value (a test build) runs that form at small n.
+#ifndef GSX_COMPACT_ONEPASS_MAX_N
+#define GSX_COMPACT_ONEPASS_MAX_N (1ll << 30)
+#endif
+static_assert(GSX_COMPACT_ONEPASS_MAX_N >= 1 && GSX_COMPACT_ONEPASS_MAX_N <= (1ll << 30),
+              "look-back words hold 30-bit survivor counts");
 #if GSX_COMPACT_ONEPASS
 constexpr int kOpThreads = 256, kOpPer = 8, kOpTile = kOpThreads * kOpPer;   // 2048 rows per tile
 constexpr uint32_t kLbAgg = 1u << 30, kLbInc = 1u << 31, kLbVal = (1u << 30) - 1u;
@@ -177,6 +186,7 @@ int compact_points(const uint8_t* mask, int64_t n, const float* xyz, const float
                    float* xyz_out, float* opacity_out, int32_t* idx_out, int64_t* count_host, void* ws,
                    int64_t ws_bytes, cudaStream_t st) {
     GSX_NVTX("gsx::compact_points");
+    GSX_REQUIRE(n >= 0 && n < GSX_N_LIMIT, GSX_ERR_ARG, "compact: n=%lld out of range [0, 2^31-64)", (long long)n);
     if (n == 0) {
         *count_host = 0;
         return GSX_OK;
@@ -184,7 +194,7 @@ int compact_points(const uint8_t* mask, int64_t n, const float* xyz, const float
     GSX_REQUIRE(ws_bytes >= compact_workspace_bytes(n), GSX_ERR_WORKSPACE, "compact: workspace too small");
     GSX_REQUIRE((opacity == nullptr) == (opacity_out == nullptr), GSX_ERR_ARG, "compact: opacity in/out mismatch");
 #if GSX_COMPACT_ONEPASS
-    {
+    if (n < GSX_COMPACT_ONEPASS_MAX_N) {
         const int64_t tiles = (n + kOpTile - 1) / kOpTile;   // (fits the two-pass workspace: fewer tiles than blocks)
         uint32_t* words = (uint32_t*)ws;                      // [0] tile counter, [1] total, [16 ..] look-back words
         GSX_CUDA_CHECK(cudaMemsetAsync(words, 0, (size_t)(tiles + 16) * 4, st));

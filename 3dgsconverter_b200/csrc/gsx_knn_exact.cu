@@ -12,6 +12,7 @@
 // 32 / 1024 / 32768 / 1048576 sorted points; one warp per query walks the 4-level hierarchy nearest
 // box first and prunes with lb >= tau, where lb is evaluated with the same monotone float64 op
 // sequence as d^2 (so lb <= d^2 of every point in the box, exactly).
+#include "../../include/gsx.h"
 #include "gsx_common.cuh"
 #include "gsx_knn_exact.cuh"
 #include "gsx_sor.cuh"
@@ -301,7 +302,7 @@ __global__ void __launch_bounds__(256, 4)
 
 int knn_exact_mean_dists(const float* xyz, int64_t n, int k, float* means, void* ws, int64_t ws_bytes,
                          cudaStream_t st) {
-    GSX_REQUIRE(n >= 1 && n < 2147483584ll, GSX_ERR_ARG, "knn_exact: n out of range");
+    GSX_REQUIRE(n >= 1 && n < GSX_N_LIMIT, GSX_ERR_ARG, "knn_exact: n out of range");
     GSX_REQUIRE(k >= 1 && k <= 63, GSX_ERR_UNSUPPORTED, "knn_exact: k must be in [1,63] (got %d)", k);
     ExWs w = ex_carve(ws, (size_t)ws_bytes, n, ex_sort_ws_bytes(n));
     GSX_REQUIRE(w.ok, GSX_ERR_WORKSPACE, "knn_exact: workspace too small");

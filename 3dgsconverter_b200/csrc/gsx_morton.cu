@@ -13,6 +13,7 @@
 //                      float32 matrix over consecutive chunks of the (optionally permuted) rows.
 // Float arithmetic of the codes follows NumPy-2 float32 semantics: (c - min) * (1024.0 / len), clip to [0,1023],
 // truncation to uint32.
+#include "../../include/gsx.h"
 #include "gsx_common.cuh"
 #include "gsx_morton.cuh"
 #include "gsx_radix.cuh"
@@ -184,7 +185,7 @@ int64_t morton_workspace_bytes(int64_t n) {
 int morton_order(const float* xyz, int64_t n, int32_t* order, int limit, int max_levels, int* levels_out, void* ws,
                  int64_t ws_bytes, cudaStream_t st) {
     GSX_NVTX("gsx::morton_order");
-    GSX_REQUIRE(n >= 0 && n < 2147483584ll, GSX_ERR_ARG, "morton: n out of range");
+    GSX_REQUIRE(n >= 0 && n < GSX_N_LIMIT, GSX_ERR_ARG, "morton: n out of range");
     if (levels_out) *levels_out = 0;
     if (n == 0) return GSX_OK;
     GSX_REQUIRE(limit >= 1, GSX_ERR_ARG, "morton: limit must be >= 1");

@@ -3,7 +3,8 @@
 // Serves the hash-grid build (gpu_ops.py:227 `np.argsort(hashed)`; word = bucket | Morton code | index, keys only)
 // and, as (key, value) pairs, the Morton orderings of the exact-KNN path and of compressed_ply / ksplat and the SOG
 // lexsort.  8-bit digits.  Two forms of a pass: the onesweep form further down is the one used (see there); the
-// three-kernel form is kept for n >= 2^30 and as the A/B baseline (-DGSX_RADIX_ONESWEEP=0):
+// three-kernel form takes over from n = GSX_RADIX_ONESWEEP_MAX_N (2^30: the onesweep look-back words carry 30-bit
+// counts) up to its own limit n < 2^32 (32-bit offsets), and is the A/B baseline (-DGSX_RADIX_ONESWEEP=0):
 //   k_rs_hist    per-tile digit histogram (tile = 4096 keys, one CTA)  -> hist[digit][tile]
 //   exclusive scan of the digit-major matrix (multi-level block scan)   -> global base of (digit, tile)
 //   k_rs_scatter per-tile stable ranks: every warp owns 512 consecutive keys, ranks them 32 at a time
@@ -21,6 +22,14 @@ namespace gsx {
 #ifndef GSX_RADIX_ONESWEEP
 #define GSX_RADIX_ONESWEEP 1
 #endif
+// onesweep sorts n < GSX_RADIX_ONESWEEP_MAX_N, the three-kernel passes everything above.  2^30 is the most the 30-bit
+// count field of a look-back word can hold; a smaller value (a test build) runs the three-kernel passes at small n.
+#ifndef GSX_RADIX_ONESWEEP_MAX_N
+#define GSX_RADIX_ONESWEEP_MAX_N (1ll << 30)
+#endif
+static_assert(GSX_RADIX_ONESWEEP_MAX_N >= 1 && GSX_RADIX_ONESWEEP_MAX_N <= (1ll << 30),
+              "onesweep look-back words hold 30-bit counts");
+constexpr int64_t kRsMaxN = 1ll << 32;   // three-kernel passes: 32-bit histogram entries and scatter offsets
 constexpr int kRsThreads = 256;
 constexpr int kRsPerThread = 16;
 constexpr int kRsTile = kRsThreads * kRsPerThread;  // 4096
@@ -117,19 +126,24 @@ __global__ void __launch_bounds__(kRsThreads) k_rs_hist(const uint64_t* __restri
     hist[(size_t)threadIdx.x * ntiles + blockIdx.x] = sh[threadIdx.x];
 }
 
-// dynamic shared memory of k_rs_scatter: the tile's pairs in locally sorted order + counters
-constexpr size_t kRsScatterSmem = (size_t)kRsTile * 12 + (size_t)8 * 256 * 4 + 2 * 256 * 4;
+// dynamic shared memory of k_rs_scatter: the tile's pairs (PAIRS = false: bare keys) in locally sorted order + counters
+template <bool PAIRS>
+constexpr size_t rs_scatter_smem() {
+    return (size_t)kRsTile * (PAIRS ? 12 : 8) + (size_t)8 * 256 * 4 + 2 * 256 * 4;
+}
 
+template <bool PAIRS>
 __global__ void __launch_bounds__(kRsThreads)
     k_rs_scatter(const uint64_t* __restrict__ keys_in, const int32_t* __restrict__ vals_in,
                  uint64_t* __restrict__ keys_out, int32_t* __restrict__ vals_out, int64_t n, int shift,
                  int64_t ntiles, const uint32_t* __restrict__ base_off) {
     extern __shared__ __align__(16) unsigned char rs_smem[];
     uint64_t* skeys = reinterpret_cast<uint64_t*>(rs_smem);                      // [kRsTile]
-    int32_t* svals = reinterpret_cast<int32_t*>(rs_smem + (size_t)kRsTile * 8);  // [kRsTile]
-    uint32_t(*wcnt)[256] = reinterpret_cast<uint32_t(*)[256]>(rs_smem + (size_t)kRsTile * 12);  // [8][256]
-    uint32_t* dstart = reinterpret_cast<uint32_t*>(rs_smem + (size_t)kRsTile * 12 + 8 * 256 * 4);  // [256]
-    uint32_t* gbase = dstart + 256;                                                                 // [256]
+    int32_t* svals = reinterpret_cast<int32_t*>(rs_smem + (size_t)kRsTile * 8);  // [kRsTile] (PAIRS only)
+    constexpr size_t kPairBytes = (size_t)kRsTile * (PAIRS ? 12 : 8);
+    uint32_t(*wcnt)[256] = reinterpret_cast<uint32_t(*)[256]>(rs_smem + kPairBytes);  // [8][256]
+    uint32_t* dstart = reinterpret_cast<uint32_t*>(rs_smem + kPairBytes + 8 * 256 * 4);  // [256]
+    uint32_t* gbase = dstart + 256;                                                       // [256]
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     for (int t = threadIdx.x; t < 8 * 256; t += kRsThreads) (&wcnt[0][0])[t] = 0;
     __syncthreads();
@@ -196,7 +210,7 @@ __global__ void __launch_bounds__(kRsThreads)
             const uint32_t d = (uint32_t)(key[e] >> shift) & 255u;
             const uint32_t lp = dstart[d] + wcnt[w][d] + rank[e];
             skeys[lp] = key[e];
-            svals[lp] = vals_in[i];
+            if (PAIRS) svals[lp] = vals_in[i];
         }
     }
     __syncthreads();
@@ -207,7 +221,7 @@ __global__ void __launch_bounds__(kRsThreads)
         const uint32_t d = (uint32_t)(k >> shift) & 255u;
         const uint32_t pos = gbase[d] + ((uint32_t)j - dstart[d]);
         keys_out[pos] = k;
-        vals_out[pos] = svals[j];
+        if (PAIRS) vals_out[pos] = svals[j];
     }
 }
 
@@ -429,22 +443,14 @@ size_t radix_ws_bytes(int64_t n) {
     return (three_kernel > onesweep ? three_kernel : onesweep) * sizeof(uint32_t);
 }
 
-int radix_sort_pairs(uint64_t* keys0, uint64_t* keys1, int32_t* vals0, int32_t* vals1, int64_t n, int begin_bit,
-                     int end_bit, void* ws, size_t ws_bytes, uint64_t** keys_sorted, int32_t** vals_sorted,
-                     cudaStream_t st) {
-    GSX_NVTX("gsx::radix_sort_pairs");
-    GSX_REQUIRE(n >= 1 && n < 4294967296ll, GSX_ERR_ARG, "radix: n out of range");
-    GSX_REQUIRE(ws_bytes >= radix_ws_bytes(n), GSX_ERR_WORKSPACE, "radix: workspace too small");
-    GSX_REQUIRE(begin_bit >= 0 && end_bit <= 64 && begin_bit < end_bit, GSX_ERR_ARG, "radix: bad bit range");
-    // onesweep whenever the look-back words can hold the counts (30 bits) -- GSX_RADIX_ONESWEEP=0 builds keep the
-    // three-kernel passes for the A/B in profiles/
-    if (GSX_RADIX_ONESWEEP && n < (1ll << 30))
-        return onesweep_sort<true>(keys0, keys1, vals0, vals1, n, begin_bit, end_bit, (uint32_t*)ws, keys_sorted,
-                                   vals_sorted, st);
+template <bool PAIRS>
+static int three_kernel_sort(uint64_t* keys0, uint64_t* keys1, int32_t* vals0, int32_t* vals1, int64_t n, int begin_bit,
+                             int end_bit, void* ws, uint64_t** keys_sorted, int32_t** vals_sorted, cudaStream_t st) {
     const int64_t ntiles = (n + kRsTile - 1) / kRsTile;
     uint32_t* hist = (uint32_t*)ws;
     uint32_t* scan_ws = hist + (size_t)256 * ntiles;
-    GSX_CUDA_CHECK(cudaFuncSetAttribute(k_rs_scatter, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRsScatterSmem));
+    GSX_CUDA_CHECK(cudaFuncSetAttribute(k_rs_scatter<PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)rs_scatter_smem<PAIRS>()));
     uint64_t *kin = keys0, *kout = keys1;
     int32_t *vin = vals0, *vout = vals1;
     for (int shift = begin_bit; shift < end_bit; shift += 8) {
@@ -452,7 +458,8 @@ int radix_sort_pairs(uint64_t* keys0, uint64_t* keys1, int32_t* vals0, int32_t* 
         GSX_KERNEL_CHECK();
         int rc = exclusive_scan_u32(hist, (int64_t)256 * ntiles, scan_ws, st);
         if (rc) return rc;
-        k_rs_scatter<<<(unsigned)ntiles, kRsThreads, kRsScatterSmem, st>>>(kin, vin, kout, vout, n, shift, ntiles, hist);
+        k_rs_scatter<PAIRS><<<(unsigned)ntiles, kRsThreads, rs_scatter_smem<PAIRS>(), st>>>(kin, vin, kout, vout, n,
+                                                                                             shift, ntiles, hist);
         GSX_KERNEL_CHECK();
         uint64_t* tk = kin;
         kin = kout;
@@ -462,18 +469,34 @@ int radix_sort_pairs(uint64_t* keys0, uint64_t* keys1, int32_t* vals0, int32_t* 
         vout = tv;
     }
     *keys_sorted = kin;
-    *vals_sorted = vin;
+    if (vals_sorted) *vals_sorted = vin;
     return GSX_OK;
+}
+
+int radix_sort_pairs(uint64_t* keys0, uint64_t* keys1, int32_t* vals0, int32_t* vals1, int64_t n, int begin_bit,
+                     int end_bit, void* ws, size_t ws_bytes, uint64_t** keys_sorted, int32_t** vals_sorted,
+                     cudaStream_t st) {
+    GSX_NVTX("gsx::radix_sort_pairs");
+    GSX_REQUIRE(n >= 1 && n < kRsMaxN, GSX_ERR_ARG, "radix: n out of range");
+    GSX_REQUIRE(ws_bytes >= radix_ws_bytes(n), GSX_ERR_WORKSPACE, "radix: workspace too small");
+    GSX_REQUIRE(begin_bit >= 0 && end_bit <= 64 && begin_bit < end_bit, GSX_ERR_ARG, "radix: bad bit range");
+    // GSX_RADIX_ONESWEEP=0 builds keep the three-kernel passes at every n for the A/B in profiles/
+    if (GSX_RADIX_ONESWEEP && n < GSX_RADIX_ONESWEEP_MAX_N)
+        return onesweep_sort<true>(keys0, keys1, vals0, vals1, n, begin_bit, end_bit, (uint32_t*)ws, keys_sorted,
+                                   vals_sorted, st);
+    return three_kernel_sort<true>(keys0, keys1, vals0, vals1, n, begin_bit, end_bit, ws, keys_sorted, vals_sorted, st);
 }
 
 int radix_sort_keys(uint64_t* keys0, uint64_t* keys1, int64_t n, int begin_bit, int end_bit, void* ws, size_t ws_bytes,
                     uint64_t** keys_sorted, cudaStream_t st) {
     GSX_NVTX("gsx::radix_sort_keys");
-    GSX_REQUIRE(n >= 1 && n < (1ll << 30), GSX_ERR_ARG, "radix: n out of range");
+    GSX_REQUIRE(n >= 1 && n < kRsMaxN, GSX_ERR_ARG, "radix: n out of range");
     GSX_REQUIRE(ws_bytes >= radix_ws_bytes(n), GSX_ERR_WORKSPACE, "radix: workspace too small");
     GSX_REQUIRE(begin_bit >= 0 && end_bit <= 64 && begin_bit < end_bit, GSX_ERR_ARG, "radix: bad bit range");
-    return onesweep_sort<false>(keys0, keys1, nullptr, nullptr, n, begin_bit, end_bit, (uint32_t*)ws, keys_sorted, nullptr,
-                                st);
+    if (n < GSX_RADIX_ONESWEEP_MAX_N)
+        return onesweep_sort<false>(keys0, keys1, nullptr, nullptr, n, begin_bit, end_bit, (uint32_t*)ws, keys_sorted,
+                                    nullptr, st);
+    return three_kernel_sort<false>(keys0, keys1, nullptr, nullptr, n, begin_bit, end_bit, ws, keys_sorted, nullptr, st);
 }
 
 }  // namespace gsx

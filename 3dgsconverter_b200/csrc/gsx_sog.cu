@@ -7,6 +7,7 @@
 // 64-bit key x:y -- after mapping floats to order-preserving unsigned ints (-0.0 is folded into +0.0 because
 // NumPy compares them equal).  quantize: lower_bound in the (<= 4096-entry) codebook held in shared memory,
 // clip, then the reference's left-neighbour test |v - cb[left]| < |v - cb[idx]| in float32.
+#include "../../include/gsx.h"
 #include "gsx_common.cuh"
 #include "gsx_radix.cuh"
 #include "gsx_sog.cuh"
@@ -42,7 +43,7 @@ int64_t lexsort_workspace_bytes(int64_t n) {
 
 int lexsort_zyx(const float* xyz, int64_t n, int32_t* order_out, void* ws, int64_t ws_bytes, cudaStream_t st) {
     if (n == 0) return GSX_OK;
-    GSX_REQUIRE(n < 2147483584ll, GSX_ERR_ARG, "lexsort: n out of range");
+    GSX_REQUIRE(n < GSX_N_LIMIT, GSX_ERR_ARG, "lexsort: n out of range");
     GSX_REQUIRE(ws_bytes >= lexsort_workspace_bytes(n), GSX_ERR_WORKSPACE, "lexsort: workspace too small");
     Carver c(ws, (size_t)ws_bytes);
     uint64_t* k0 = c.take<uint64_t>((size_t)n);

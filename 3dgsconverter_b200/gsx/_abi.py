@@ -113,5 +113,12 @@ def check(rc: int, what: str = ""):
         raise GsxError(f"{what or 'gsx'} failed (status {rc}): {msg}")
 
 
+def workspace_size(name: str, *args) -> int:
+    """Byte size from a *_workspace_bytes entry point; a negative result (n out of range) raises GsxError."""
+    nbytes = getattr(lib, name)(*args)
+    check(nbytes if nbytes < 0 else 0, name)
+    return nbytes
+
+
 def f32x(*vals):
     return (C.c_float * len(vals))(*[float(v) for v in vals])

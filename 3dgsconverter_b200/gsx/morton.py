@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 import torch
 
-from ._abi import lib, check
+from ._abi import lib, check, workspace_size
 from .sor import _ptr, _stream, _check_xyz
 
 
@@ -16,7 +16,7 @@ def morton_order(xyz: torch.Tensor, run_limit: int = 256, return_levels: bool = 
     _check_xyz(xyz)
     n = xyz.shape[0]
     order = torch.empty(n, dtype=torch.int32, device=xyz.device)
-    ws = torch.empty(lib.gsx_morton_workspace_bytes(n), dtype=torch.uint8, device=xyz.device)
+    ws = torch.empty(workspace_size("gsx_morton_workspace_bytes", n), dtype=torch.uint8, device=xyz.device)
     lv = C.c_int32(0)
     check(lib.gsx_morton_order(_ptr(xyz), n, _ptr(order), int(run_limit), C.byref(lv), _ptr(ws), ws.numel(), _stream()),
           "gsx_morton_order")

@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import density as _density, masks as _masks, sor as _sor
-from ._abi import lib, check
+from ._abi import lib, check, workspace_size
 from .sor import _ptr, _stream
 
 
@@ -22,7 +22,7 @@ def compact(mask: torch.Tensor, xyz: torch.Tensor, opacity: torch.Tensor | None,
     n = xyz.shape[0]
     dev = xyz.device
     m8 = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
-    ws = torch.empty(lib.gsx_compact_workspace_bytes(n), dtype=torch.uint8, device=dev)
+    ws = torch.empty(workspace_size("gsx_compact_workspace_bytes", n), dtype=torch.uint8, device=dev)
     xyz_o = torch.empty_like(xyz)
     op_o = torch.empty_like(opacity) if opacity is not None else None
     idx_o = torch.empty(n, dtype=torch.int32, device=dev)

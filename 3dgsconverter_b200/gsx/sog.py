@@ -12,7 +12,7 @@ import ctypes as C
 import numpy as np
 import torch
 
-from ._abi import lib, check
+from ._abi import lib, check, workspace_size
 from .sor import _ptr, _stream, _check_xyz
 
 
@@ -21,7 +21,7 @@ def lexsort_zyx(xyz: torch.Tensor) -> torch.Tensor:
     _check_xyz(xyz)
     n = xyz.shape[0]
     order = torch.empty(n, dtype=torch.int32, device=xyz.device)
-    ws = torch.empty(lib.gsx_lexsort_workspace_bytes(n), dtype=torch.uint8, device=xyz.device)
+    ws = torch.empty(workspace_size("gsx_lexsort_workspace_bytes", n), dtype=torch.uint8, device=xyz.device)
     check(lib.gsx_lexsort_zyx(_ptr(xyz), n, _ptr(order), _ptr(ws), ws.numel(), _stream()), "gsx_lexsort_zyx")
     return order
 

@@ -45,10 +45,7 @@ class SorGrid:
 
 
 def workspace(n: int, device) -> torch.Tensor:
-    nbytes = lib.gsx_sor_workspace_bytes(n)
-    if nbytes <= 0:
-        raise _abi.GsxError("gsx_sor_workspace_bytes failed")
-    return torch.empty(nbytes, dtype=torch.uint8, device=device)
+    return torch.empty(_abi.workspace_size("gsx_sor_workspace_bytes", n), dtype=torch.uint8, device=device)
 
 
 def build_grid(xyz: torch.Tensor, ws: torch.Tensor | None = None, cell_scale: float = 1.0) -> SorGrid:
@@ -157,7 +154,7 @@ def ckdtree_mean_dists(xyz: torch.Tensor, k: int) -> torch.Tensor:
     """data_processor.py:160-173 on device: exact (k+1)-NN in float64, mean of neighbours 1..k -> float32."""
     _check_xyz(xyz)
     n = xyz.shape[0]
-    ws = torch.empty(lib.gsx_knn_exact_workspace_bytes(n), dtype=torch.uint8, device=xyz.device)
+    ws = torch.empty(_abi.workspace_size("gsx_knn_exact_workspace_bytes", n), dtype=torch.uint8, device=xyz.device)
     out = torch.empty(n, dtype=torch.float32, device=xyz.device)
     check(lib.gsx_knn_exact_mean_dists(_ptr(xyz), n, int(k), _ptr(out), _ptr(ws), ws.numel(), _stream()),
           "gsx_knn_exact_mean_dists")
@@ -189,7 +186,7 @@ def sort_pairs(keys: torch.Tensor, vals: torch.Tensor | None, begin_bit: int = 0
     """In-place stable radix sort of (int64-viewed-as-uint64 keys, int32 vals) on key bits [begin,end).
     vals=None sorts bare 64-bit words (payload packed below begin_bit), the form the grid build uses."""
     n = keys.numel()
-    ws = torch.empty(lib.gsx_sort_pairs_workspace_bytes(n), dtype=torch.uint8, device=keys.device)
+    ws = torch.empty(_abi.workspace_size("gsx_sort_pairs_workspace_bytes", n), dtype=torch.uint8, device=keys.device)
     check(lib.gsx_sort_pairs(_ptr(keys), _ptr(vals), n, begin_bit, end_bit, _ptr(ws), ws.numel(), _stream()),
           "gsx_sort_pairs")
     return keys, vals

@@ -21,7 +21,15 @@
  *     The *_host convenience entry points take host buffers and manage device memory
  *     internally (cudaMallocAsync), copies included.
  *   - all masks are uint8 (0/1), one byte per point, like numpy bool.
- *   - N < 2^31 - 64 (int32 indices, as in gpu_ops.py:224,233-234).
+ *   - N < 2^31 - 64 = GSX_N_LIMIT (int32 indices, as in gpu_ops.py:224,233-234) for every entry point that takes a
+ *     point count, except the generic gsx_sort_pairs (n < 2^32).  The *_workspace_bytes functions of those entry
+ *     points return GSX_ERR_ARG for an n outside the range.
+ *     Two primitives change algorithm at 2^30 rows, because below it they chain 30-bit running counts through
+ *     decoupled look-back words (one kernel): the radix sort (gsx_sort_pairs and every sort inside SOR, lexsort,
+ *     Morton order and the cKDTree-semantics KNN) runs onesweep passes for n < 2^30 and three-kernel
+ *     histogram / scan / scatter passes with 32-bit offsets from 2^30 on; gsx_compact_points runs one look-back pass
+ *     for n < 2^30 and count / scan / scatter from 2^30 on.  tests/test_size_limits_gpu.py runs both sides: the
+ *     shipped library at n > 2^30, and the existing small-n checks against builds whose switch-over is 4096 rows.
  */
 #ifndef GSX_H
 #define GSX_H
@@ -30,6 +38,8 @@
 #ifdef __cplusplus
 extern "C" {
 #endif
+
+#define GSX_N_LIMIT 2147483584LL /* 2^31 - 64: every point count n < GSX_N_LIMIT */
 
 #define GSX_HASH_I32WRAP 0 /* probe hash with wrapping int32 products: Taichi default_ip (faithful, SURVEY F8) */
 #define GSX_HASH_I64 1     /* probe hash with int64 products: what the host table build uses (intended) */
@@ -113,9 +123,10 @@ int gsx_sor_mean_dists_strided(int64_t n, int32_t stride, int32_t phase, int32_t
 
 /* gpu_ops.py:227 (np.argsort of the bucket hashes): stable LSD radix sort, in place, of (uint64 key, int32
  * value) pairs on the key bits [begin_bit, end_bit): 8-bit digits, one "onesweep" kernel per digit (decoupled
- * look-back over per-tile digit counts) after a single histogram pass.  vals_dev == NULL sorts bare 64-bit words
- * (n < 2^30): the form the hash-grid build uses, with word = bucket | in-cell Morton code | original index and only the
- * bits above the index sorted -- 8 instead of 12 bytes moved per point and pass. */
+ * look-back over per-tile digit counts) after a single histogram pass; from n = 2^30 on, histogram / scan / scatter
+ * kernels per digit.  vals_dev == NULL sorts bare 64-bit words: the form the hash-grid build uses, with
+ * word = bucket | in-cell Morton code | original index and only the bits above the index sorted -- 8 instead of 12
+ * bytes moved per point and pass.  1 <= n < 2^32 (n = 0 is a no-op); the workspace size is GSX_ERR_ARG above. */
 int64_t gsx_sort_pairs_workspace_bytes(int64_t n);
 int gsx_sort_pairs(uint64_t* keys_dev, int32_t* vals_dev, int64_t n, int32_t begin_bit, int32_t end_bit, void* ws,
                    int64_t ws_bytes, void* stream);
