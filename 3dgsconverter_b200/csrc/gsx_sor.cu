@@ -1059,6 +1059,41 @@ __device__ __forceinline__ void scan32(const float4* __restrict__ spos, pos_t j,
 #ifndef GSX_KNN_MINBLOCKS
 #define GSX_KNN_MINBLOCKS 8
 #endif
+// Group path (K <= 32, batched epilogue): a batch whose positions all lie in one grid cell, inside the long bucket that
+// the centre probe reaches, walks the probes / super boxes / chunk boxes ONCE for the whole batch.  The walk prunes
+// with the box-to-box bound lb(B, box) (B = bounding box of the batch) against tau_G = the largest seed tau of the
+// batch, and lists what survives; each query then tests only the listed boxes with its own bound.  Exact: for every q
+// in B, lb(B, box) <= box_lb(q, box) (same monotone op sequence), and tau_G >= every member's tau, so a box left out
+// satisfies lb(q) >= tau_seed(q) -- the same rule as the per-query walk (DESIGN §4.2).  A seed list that is not full,
+// or a list longer than GSX_KNN_GROUP_LIST entries, sends the batch to the per-query path.
+#ifndef GSX_KNN_GROUP
+#define GSX_KNN_GROUP 1
+#endif
+#ifndef GSX_KNN_GROUP_LIST
+#define GSX_KNN_GROUP_LIST 256
+#endif
+// A/B (profiles/r03_knn_variants.log, 10 M mixed): 32 / 64 entries slower than no group path, 128 -3.6 %, 256 -4.5 %,
+// 512 -2.2 % (the shared memory starts to cost L1)
+constexpr int kGroupList = GSX_KNN_GROUP_LIST;   // list entries per warp (shared memory)
+// Diagnostic build (scripts/knn_class_profile.py): with stats, lane 0 of every batch adds the batch's clock64 cycles
+// and query count to one of 4 classes by the size of the centre probe's bucket (<= 64, <= 1024, <= 16384, larger):
+// stats[8 + c] cycles, stats[12 + c] queries.  Never shipped.
+#ifndef GSX_KNN_PROFILE
+#define GSX_KNN_PROFILE 0
+#endif
+#ifndef GSX_KNN_CELLBITS
+#define GSX_KNN_CELLBITS 1
+#endif
+
+// shared memory of k_sor_knn: the epilogue rows, then (group path) one list per warp
+template <int NREG, int ES>
+__host__ __device__ constexpr bool knn_group_on() { return GSX_KNN_GROUP && GSX_KNN_CELLBITS && NREG == 1 && ES > 0; }
+template <int NREG, int ES>
+constexpr size_t knn_smem_bytes() {
+    return (size_t)8 * kQueryBatch * ES * sizeof(float) +
+           (knn_group_on<NREG, ES>() ? (size_t)8 * (kGroupList + 32) * sizeof(unsigned) : 0);
+}
+
 template <int NREG, bool STATS, int ES>
 __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
     k_sor_knn(const float4* __restrict__ spos, const int2* __restrict__ tab_se, const float4* __restrict__ tab_box,
@@ -1068,12 +1103,22 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
               float bz, float cell,
               uint32_t n, uint64_t M, unsigned long long* __restrict__ stats) {
     const int lane = lane_id();
-    unsigned long long st_visits = 0, st_scanned = 0, st_boxes = 0, st_queries = 0;
+    unsigned long long st_visits = 0, st_scanned = 0, st_boxes = 0, st_queries = 0, st_group = 0;
     static_assert(ES >= 0 && ES <= 33, "a row holds at most the 32 ranks of one register + the row number");
     // batched epilogue (ES > 0): [8 warps][kQueryBatch][ES] floats, a row = ES-1 ranks (>= K) + the row number; ES is
     // odd so that the lanes of the final pass (one query each) read distinct banks
     extern __shared__ float s_epi[];
     float* const epi = s_epi + (threadIdx.x >> 5) * (kQueryBatch * (ES > 0 ? ES : 1));
+    // group path, per warp: the list (entry = chunk id << 5 | probe; chunk ids < 2^26), then the bucket hash of probe
+    // p at glist[kGroupList + p], so that the group code can reload the probe boxes instead of keeping them live
+    constexpr bool GROUP = knn_group_on<NREG, ES>();
+    unsigned* const glist =
+        reinterpret_cast<unsigned*>(s_epi + 8 * kQueryBatch * ES) + (threadIdx.x >> 5) * (kGroupList + 32);
+    auto probe_box = [&](float& lx, float& ly, float& lz, float& hx, float& hy, float& hz) {   // lane < 27, pc > 0
+        const size_t h = glist[kGroupList + lane];
+        const float4 b0 = __ldg(tab_box + 2 * h), b1 = __ldg(tab_box + 2 * h + 1);
+        lx = b0.x, ly = b0.y, lz = b0.z, hx = b1.x, hy = b1.y, hz = b1.z;
+    };
 #if GSX_KNN_TMA
     __shared__ __align__(128) float4 s_stage[8][kSmallBucket];
     __shared__ __align__(8) unsigned long long s_bar[8];
@@ -1084,10 +1129,12 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
     if (lane == 0) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_addr) : "memory");
     __syncwarp();
 #endif
-    // probe offsets of lane p<27 in the reference's loop order (dx outer, dz inner)
-    const int pdx = lane / 9 - 1, pdy = (lane / 3) % 3 - 1, pdz = lane % 3 - 1;
 
     for (;;) {
+#if GSX_KNN_PROFILE
+        const long long prof_t0 = clock64();
+        int prof_cls = 0;
+#endif
         unsigned int b0 = 0;
         if (lane == 0) b0 = atomicAdd(work, (unsigned)kQueryBatch);
         b0 = __shfl_sync(GSX_FULL, b0, 0);
@@ -1098,9 +1145,6 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
         int64_t qe = qb + kQueryBatch < q_end ? qb + kQueryBatch : q_end;
         // the 27 probes of a query depend only on its cell: consecutive hash-sorted queries mostly share
         // it, so the hashes and table entries are recomputed only when the cell changes
-#ifndef GSX_KNN_CELLBITS
-#define GSX_KNN_CELLBITS 1
-#endif
 #if GSX_KNN_CELLBITS
         // one bit per sorted position (k_sor_finish): "another grid cell than the position before".  A batch is 16
         // consecutive positions inside one 32-bit word (kQueryBatch divides 32, batches are aligned to q_begin).
@@ -1113,7 +1157,7 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
         const pos_t qb_p = (pos_t)qb, qe_p = (pos_t)qe;      // positions fit 31 bits (pos_t): 32-bit loop bookkeeping
 #pragma unroll 1
         for (pos_t i = qb_p; i < qe_p; ++i) {
-            const float4 q = __ldg(spos + i);
+            float4 q = __ldg(spos + i);
 #if GSX_KNN_CELLBITS
             const uint32_t w_i = (i >> 5) == (qb_p >> 5) ? cellword : __ldg(cellbits + (i >> 5));
             if (i == qb_p || ((w_i >> (i & 31)) & 1u)) {   // warp-uniform by construction
@@ -1133,7 +1177,13 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
 #endif
                 ps = 0, pc = 0;
                 if (lane < 27) {
+                    // probe offsets of lane p<27 in the reference's loop order (dx outer, dz inner), computed here
+                    // rather than held in registers through the query
+                    unsigned pl;
+                    asm volatile("mov.u32 %0, %%laneid;" : "=r"(pl));   // volatile: not hoisted out of the loop
+                    const int pdx = (int)pl / 9 - 1, pdy = ((int)pl / 3) % 3 - 1, pdz = (int)pl % 3 - 1;
                     uint32_t h = probe_hash(gx + pdx, gy + pdy, gz + pdz, n, M, hash_mode);
+                    if (GROUP) glist[kGroupList + lane] = h;
                     const int2 se = __ldg(tab_se + h);
                     ps = se.x;
                     pc = se.y - se.x;
@@ -1175,6 +1225,191 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
                 }
 #endif
             }
+#if GSX_KNN_PROFILE
+            if (i == qb_p) {
+                const int c13 = __shfl_sync(GSX_FULL, pc, 13);
+                prof_cls = c13 <= kSmallBucket ? 0 : c13 <= 1024 ? 1 : c13 <= 16384 ? 2 : 3;
+            }
+#endif
+#if GSX_KNN_CELLBITS
+            if constexpr (GROUP) if (i == qb_p) {
+                const int s13 = __shfl_sync(GSX_FULL, ps, 13), c13 = __shfl_sync(GSX_FULL, pc, 13);
+                const pos_t ql = qe_p - 1;
+                // positions qb+1 .. qe-1 of the cell word: a set bit = another cell than the position before
+                const uint32_t later = ((2u << (ql & 31)) - 1u) & ~((2u << (qb_p & 31)) - 1u);
+                if (c13 > kSmallBucket && qb_p >= s13 && qe_p <= (pos_t)s13 + c13 && (ql >> 5) == (qb_p >> 5) &&
+                    (cellword & later) == 0u) {
+                    // phase A: the seed list of every query (its own chunk, as the per-query path does), parked in
+                    // the query's epilogue row; B = box of the batch, tau_G = largest seed tau
+                    const int skip_chunk = (int)(qb_p >> 5);
+                    const pos_t js = ((pos_t)skip_chunk << 5) + lane;
+                    const bool jv = js >= s13 && js < (pos_t)s13 + c13;
+                    float tau_g = 0.f;
+                    float Blx = INFINITY, Bly = INFINITY, Blz = INFINITY, Bhx = -INFINITY, Bhy = -INFINITY,
+                          Bhz = -INFINITY;
+                    bool full = true;
+#pragma unroll 1
+                    for (pos_t t = qb_p; t < qe_p; ++t) {
+                        const float4 qt = __ldg(spos + t);
+                        TopK<NREG> tk;
+                        tk.init(K);
+                        scan32<NREG, STATS>(spos, js, jv, qt.x, qt.y, qt.z, tk, lane, st_scanned);
+                        if (!(tk.tau < __uint_as_float(GSX_D2LIM_BITS))) {   // fewer than K candidates in the chunk
+                            full = false;
+                            break;
+                        }
+                        tau_g = fmaxf(tau_g, tk.tau);
+                        Blx = fminf(Blx, qt.x), Bly = fminf(Bly, qt.y), Blz = fminf(Blz, qt.z);
+                        Bhx = fmaxf(Bhx, qt.x), Bhy = fmaxf(Bhy, qt.y), Bhz = fmaxf(Bhz, qt.z);
+                        if (lane < ES - 1) epi[(int)(t - qb_p) * ES + lane] = tk.v0;
+                    }
+                    // phase B: one walk for the batch.  The bound per axis is max(lo_box - hi_B, lo_B - hi_box, 0),
+                    // then the op sequence of box_lb: <= box_lb(q, box) for every q in B.
+                    auto lb_b = [&](float lx, float ly, float lz, float hx, float hy, float hz) {
+                        const float dx = fmaxf(fmaxf(__fsub_rn(lx, Bhx), __fsub_rn(Blx, hx)), 0.f);
+                        const float dy = fmaxf(fmaxf(__fsub_rn(ly, Bhy), __fsub_rn(Bly, hy)), 0.f);
+                        const float dz = fmaxf(fmaxf(__fsub_rn(lz, Bhz), __fsub_rn(Blz, hz)), 0.f);
+                        return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
+                    };
+                    int cnt = 0;
+                    auto append = [&](bool take, unsigned entry) {   // ballot compaction into the warp's list
+                        const unsigned m = __ballot_sync(GSX_FULL, take);
+                        const int at = cnt + __popc(m & ((1u << lane) - 1u));
+                        if (take && at < kGroupList) glist[at] = entry;
+                        cnt += __popc(m);
+                    };
+                    unsigned small = 0;   // probes whose (small) bucket passed the group bound
+                    if (full) {
+                        // a bucket reached by two probes is listed (and later scanned) twice, as in the per-query path
+                        bool pt = false;
+                        if (pc > 0) {
+                            float lx, ly, lz, hx, hy, hz;
+                            probe_box(lx, ly, lz, hx, hy, hz);
+                            pt = lb_b(lx, ly, lz, hx, hy, hz) < tau_g;
+                        }
+                        small = __ballot_sync(GSX_FULL, pt && pc <= kSmallBucket);
+                        unsigned lm = __ballot_sync(GSX_FULL, pt && pc > kSmallBucket);
+                        while (lm && cnt <= kGroupList) {
+                            const int p = __ffs(lm) - 1;
+                            lm &= lm - 1;
+                            const int s = __shfl_sync(GSX_FULL, ps, p), c = __shfl_sync(GSX_FULL, pc, p);
+                            const int fc = s >> 5, lc = (s + c - 1) >> 5, fs = fc >> 5, ls = lc >> 5;
+                            auto chunks = [&](const int cbase) {
+                                const int cid = cbase + lane;
+                                bool take = false;
+                                if (cid >= fc && cid <= lc) {
+                                    const float4 a = __ldg(caabb + 2 * cid), b = __ldg(caabb + 2 * cid + 1);
+                                    take = lb_b(a.x, a.y, a.z, a.w, b.x, b.y) < tau_g;
+                                }
+                                if (STATS) st_boxes += __popc(__ballot_sync(GSX_FULL, cid >= fc && cid <= lc));
+                                append(take, ((unsigned)cid << 5) | (unsigned)p);
+                            };
+                            if (GSX_KNN_FLAT_SUPERS > 0 && ls - fs < GSX_KNN_FLAT_SUPERS) {
+                                for (int cb = fc; cb <= lc && cnt <= kGroupList; cb += 32) chunks(cb);
+                                continue;
+                            }
+                            for (int sb = fs; sb <= ls && cnt <= kGroupList; sb += 32) {
+                                const int sid = sb + lane;
+                                bool take = false;
+                                if (sid <= ls) {
+                                    const float4 a = __ldg(saabb + 2 * sid), b = __ldg(saabb + 2 * sid + 1);
+                                    take = lb_b(a.x, a.y, a.z, a.w, b.x, b.y) < tau_g;
+                                }
+                                if (STATS) st_boxes += __popc(__ballot_sync(GSX_FULL, sid <= ls));
+                                unsigned sm = __ballot_sync(GSX_FULL, take);
+                                while (sm && cnt <= kGroupList) {
+                                    const int srcs = __ffs(sm) - 1;
+                                    sm &= sm - 1;
+                                    chunks((sb + srcs) * 32);
+                                }
+                            }
+                        }
+                    }
+                    if (full && cnt <= kGroupList) {
+                        __syncwarp();   // the list is read by other lanes than the ones that wrote it
+                        // phase C: per query, its seed list back, then the listed chunks and the small buckets, each
+                        // nearest box first
+#pragma unroll 1
+                        for (pos_t t = qb_p; t < qe_p; ++t) {
+                            const float4 qt = __ldg(spos + t);
+                            TopK<NREG> tk;
+                            tk.init(K);
+                            // ranks >= ES-1 >= K are never read: the sentinel keeps the list ascending
+                            if (lane < ES - 1) tk.v0 = epi[(int)(t - qb_p) * ES + lane];
+                            tk.refresh_tau();
+#pragma unroll 1
+                            for (int g0 = 0; g0 < cnt; g0 += 32) {
+                                const bool ev = g0 + lane < cnt;
+                                const unsigned ent = ev ? glist[g0 + lane] : 0u;
+                                unsigned key = 0xffffffffu;
+                                if (ev && ent != (((unsigned)(qb_p >> 5) << 5) | 13u)) {   // not the seed chunk
+                                    const float lb = box_lb(caabb, (int)(ent >> 5), qt.x, qt.y, qt.z);
+                                    if (lb < tk.tau) key = __float_as_uint(lb);
+                                }
+                                if (STATS) st_boxes += __popc(__ballot_sync(GSX_FULL, ev));
+                                for (;;) {
+                                    const unsigned mc = __reduce_min_sync(GSX_FULL, key);
+                                    if (mc == 0xffffffffu || !(__uint_as_float(mc) < tk.tau)) break;
+                                    const int src = __ffs(__ballot_sync(GSX_FULL, key == mc)) - 1;
+                                    if (lane == src) key = 0xffffffffu;
+                                    const unsigned e_src = __shfl_sync(GSX_FULL, ent, src);
+                                    const int pp = (int)(e_src & 31u);
+                                    const int s = __shfl_sync(GSX_FULL, ps, pp), c = __shfl_sync(GSX_FULL, pc, pp);
+                                    const pos_t j = ((pos_t)(e_src >> 5) << 5) + lane;
+                                    scan32<NREG, STATS>(spos, j, j >= s && j < (pos_t)s + c, qt.x, qt.y, qt.z, tk, lane,
+                                                        st_scanned);
+                                }
+                            }
+                            unsigned pkey = 0xffffffffu;
+                            if ((small >> lane) & 1u) {
+                                float blx, bly, blz, bhx, bhy, bhz;
+                                probe_box(blx, bly, blz, bhx, bhy, bhz);
+                                const float dx = fmaxf(fmaxf(__fsub_rn(blx, qt.x), __fsub_rn(qt.x, bhx)), 0.f);
+                                const float dy = fmaxf(fmaxf(__fsub_rn(bly, qt.y), __fsub_rn(qt.y, bhy)), 0.f);
+                                const float dz = fmaxf(fmaxf(__fsub_rn(blz, qt.z), __fsub_rn(qt.z, bhz)), 0.f);
+                                pkey = __float_as_uint(
+                                    __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
+                            }
+#pragma unroll 1
+                            for (;;) {
+                                const unsigned mp = __reduce_min_sync(GSX_FULL, pkey);
+                                if (mp == 0xffffffffu || !(__uint_as_float(mp) < tk.tau)) break;
+                                const int p = __ffs(__ballot_sync(GSX_FULL, pkey == mp)) - 1;
+                                if (lane == p) pkey = 0xffffffffu;
+                                const int s = __shfl_sync(GSX_FULL, ps, p), c = __shfl_sync(GSX_FULL, pc, p);
+                                const pos_t e = (pos_t)s + c;
+#pragma unroll 1
+                                for (pos_t base = s; base < e; base += 32)
+                                    scan32<NREG, STATS>(spos, base + lane, base + lane < e, qt.x, qt.y, qt.z, tk, lane,
+                                                        st_scanned);
+                            }
+                            const float d0 = __fsqrt_rn(tk.v0);
+                            float* row = epi + (int)(t - qb_p) * ES;
+                            if (ES <= 32) {
+                                if (lane < ES) row[lane] = lane == ES - 1 ? qt.w : d0;
+                            } else {
+                                row[lane] = d0;
+                                if (lane == 0) row[ES - 1] = qt.w;
+                            }
+                        }
+                        if (STATS) {
+                            int tot = pc;
+#pragma unroll
+                            for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(GSX_FULL, tot, o);
+                            st_visits += (unsigned long long)tot * (unsigned long long)(qe_p - qb_p);
+                            st_queries += (unsigned long long)(qe_p - qb_p);
+                            st_group += (unsigned long long)(qe_p - qb_p);
+                        }
+                        break;   // the batched epilogue below sums the rows
+                    }
+                    // fallback to the per-query path: q and the probe boxes are reloaded, so that they are not live
+                    // through the group code
+                    q = __ldg(spos + i);
+                    blx = bly = blz = bhx = bhy = bhz = 0.f;
+                    if (lane < 27 && pc > 0) probe_box(blx, bly, blz, bhx, bhy, bhz);
+                }
+            }
+#endif
             if (STATS) {
                 int tot = pc;
 #pragma unroll
@@ -1305,7 +1540,7 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
         }
         if (ES > 0) {
             __syncwarp();
-            if (lane < (int)(qe - qb)) {   // lane q: the serial sum of query q, rank order, exactly as above
+            if (lane < (int)(qe_p - qb_p)) {   // lane q: the serial sum of query q, rank order, exactly as above
                 const float* row = epi + lane * ES;
                 float sum = 0.f;
                 int valid = 0;
@@ -1318,14 +1553,21 @@ __global__ void __launch_bounds__(256, GSX_KNN_MINBLOCKS)
                 }
                 final_means[__float_as_int(row[ES - 1])] = valid > 0 ? __fdiv_rn(sum, (float)valid) : 0.f;
             }
-            __syncwarp();   // the next batch overwrites the rows
+            __syncwarp();   // the next batch overwrites the rows (and the group list)
         }
+#if GSX_KNN_PROFILE
+        if (STATS && lane == 0) {
+            atomicAdd(stats + 8 + prof_cls, (unsigned long long)(clock64() - prof_t0));
+            atomicAdd(stats + 12 + prof_cls, (unsigned long long)(qe_p - qb_p));
+        }
+#endif
     }
     if (STATS && lane == 0) {
         atomicAdd(stats + 0, st_visits);
         atomicAdd(stats + 1, st_scanned);
         atomicAdd(stats + 2, st_boxes);
         atomicAdd(stats + 3, st_queries);
+        atomicAdd(stats + 4, st_group);
     }
 }
 
@@ -1345,7 +1587,7 @@ static int launch_knn(SorWs& w, int64_t q_begin, int64_t q_end, int q_stride, in
                       const float* bmin, float cell,
                       float* final_means, unsigned long long* stats, uint64_t M, int64_t want, cudaStream_t st) {
     int per_sm = 0;
-    const size_t smem = (size_t)8 * kQueryBatch * ES * sizeof(float);
+    const size_t smem = knn_smem_bytes<NREG, ES>();
     GSX_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_sor_knn<NREG, STATS, ES>, 256, smem));
     int64_t grid = (int64_t)sm_count() * (per_sm > 0 ? per_sm : 4);  // persistent: exactly the resident CTAs
     if (grid > want) grid = want;
@@ -1383,7 +1625,8 @@ static int launch_knn16(SorWs& w, int64_t q_begin, int64_t q_end, int q_stride, 
 #define GSX_FLAT_INFO ""
 #endif
 const char* sor_build_info() {
-    return "knn=r02c"
+    return "knn=r03"
+           ";group=" GSX_STR(GSX_KNN_GROUP) ";group_list=" GSX_STR(GSX_KNN_GROUP_LIST) ";profile=" GSX_STR(GSX_KNN_PROFILE)
            ";epi_smem=" GSX_STR(GSX_KNN_EPI_SMEM) ";first_sort=" GSX_STR(GSX_KNN_FIRST_SORT)
            ";query_batch=" GSX_STR(GSX_QUERY_BATCH) ";minblocks=" GSX_STR(GSX_KNN_MINBLOCKS)
            ";merge_threshold=" GSX_STR(GSX_MERGE_THRESHOLD) ";small_bucket=" GSX_STR(GSX_SMALL_BUCKET)

@@ -69,21 +69,27 @@ def build_grid(xyz: torch.Tensor, ws: torch.Tensor | None = None, cell_scale: fl
     return SorGrid(n, ws, bmin, cell)
 
 
+def _stats_dict(v) -> dict:
+    """The 16 counters of gsx_sor_mean_dists (gsx.h); class_cycles / class_queries are zero unless the library was
+    built with -DGSX_KNN_PROFILE=1."""
+    return dict(visits=int(v[0]), scanned=int(v[1]), box_tests=int(v[2]), queries=int(v[3]), group_queries=int(v[4]),
+                class_cycles=[int(x) for x in v[8:12]], class_queries=[int(x) for x in v[12:16]])
+
+
 def mean_dists(grid: SorGrid, k: int, hash_mode: str | None = None, out: torch.Tensor | None = None,
                want_stats: bool = False, q_range: tuple[int, int] | None = None):
-    """gpu_ops.py:98-176 + unsort (:255-256).  Returns final_means (and the 4 counters if asked)."""
+    """gpu_ops.py:98-176 + unsort (:255-256).  Returns final_means (and the counters if asked)."""
     mode = HASH_MODES[hash_mode or default_hash_mode()]
     dev = grid.ws.device
     if out is None:
         out = torch.empty(grid.n, dtype=torch.float32, device=dev)
-    stats = torch.zeros(4, dtype=torch.int64, device=dev) if want_stats else None
+    stats = torch.zeros(16, dtype=torch.int64, device=dev) if want_stats else None
     qb, qe = q_range if q_range is not None else (0, grid.n)
     check(lib.gsx_sor_mean_dists_range(grid.n, qb, qe, int(k), mode, grid.bmin.ctypes.data_as(C.POINTER(C.c_float)),
                                        grid.cell, _ptr(grid.ws), grid.ws.numel(), _ptr(out), _ptr(stats), _stream()),
           "gsx_sor_mean_dists")
     if want_stats:
-        v = stats.cpu().numpy()
-        return out, dict(visits=int(v[0]), scanned=int(v[1]), box_tests=int(v[2]), queries=int(v[3]))
+        return out, _stats_dict(stats.cpu().numpy())
     return out
 
 
@@ -91,13 +97,12 @@ def mean_dists_strided(grid: SorGrid, k: int, hash_mode: str | None, out: torch.
                        want_stats: bool = False):
     """Queries the 16-position batches b with b % stride == phase (cost-balanced multi-GPU sharding)."""
     mode = HASH_MODES[hash_mode or default_hash_mode()]
-    stats = torch.zeros(4, dtype=torch.int64, device=out.device) if want_stats else None
+    stats = torch.zeros(16, dtype=torch.int64, device=out.device) if want_stats else None
     check(lib.gsx_sor_mean_dists_strided(grid.n, int(stride), int(phase), int(k), mode,
                                          grid.bmin.ctypes.data_as(C.POINTER(C.c_float)), grid.cell, _ptr(grid.ws),
                                          grid.ws.numel(), _ptr(out), _ptr(stats), _stream()), "gsx_sor_mean_dists_strided")
     if want_stats:
-        v = stats.cpu().numpy()
-        return out, dict(visits=int(v[0]), scanned=int(v[1]), box_tests=int(v[2]), queries=int(v[3]))
+        return out, _stats_dict(stats.cpu().numpy())
     return out
 
 

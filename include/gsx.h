@@ -102,8 +102,10 @@ int gsx_sor_build_from_sorted(const float* spos4_dev, const uint8_t* flags_dev /
 
 /* gpu_ops.py:98-176 + :255-256: K = min(k,50) nearest candidates over the 27 probed buckets, mean of
  * their distances, written in the caller's point order (the "unsort" is fused).  Must follow
- * gsx_sor_build on the same workspace.  hash_mode = GSX_HASH_*.  stats_dev (may be NULL) receives
- * 4 uint64 counters {reference-model visits V, candidates actually scanned, box tests, queries}. */
+ * gsx_sor_build on the same workspace.  hash_mode = GSX_HASH_*.  stats_dev (may be NULL, else 16 zeroed uint64)
+ * accumulates {reference-model visits V, candidates actually scanned, box tests, queries, queries answered by the
+ * group path, 0, 0, 0, then 4 cycle counts and 4 query counts per class of centre-bucket size (<= 64, <= 1024,
+ * <= 16384, larger) -- these 8 only in a -DGSX_KNN_PROFILE=1 build}. */
 int gsx_sor_mean_dists(int64_t n, int32_t k, int32_t hash_mode, const float* bmin_host, float cell, void* ws,
                        int64_t ws_bytes, float* final_means_dev, unsigned long long* stats_dev, void* stream);
 
